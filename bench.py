@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — audio-seconds per wall-second of the Whisper hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                  # this engine
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this engine
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] # the reference's own CPU path on the host cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # N > 1, one rank per GPU
 
@@ -60,7 +60,12 @@ def parse_args():
     ap.add_argument("--chunk-base", type=int, default=-1, help="debug: use synthetic chunks base .. base+B-1 instead of the fixture's (no token check)")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the reference CPU leg (model sweeps; the default run keeps it)")
     ap.add_argument("--ref-tokens", type=int, default=12, help="reference arm: decoder tokens actually run per sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (greedy tokens, last-step logits) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def workload_name(a):
@@ -80,6 +85,26 @@ def hbm_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, prefix=""):
+    """Write each [batch][...] array as out_dir/<prefix><name>.npy in float32.  If they exceed DUMP_LIMIT_BYTES together, only a fixed,
+    seeded sample of batch rows is written (the same rows of every array), and their indices go to <prefix>rows.npy."""
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    batch = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v.nbytes // max(1, v.shape[0]) for v in arrays.values())
+    if row_bytes * batch > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // (row_bytes + 4))        # + the row's index in rows.npy
+        rows = np.sort(np.random.default_rng(0).choice(batch, keep, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows.astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, prefix + k + ".npy"), v)
+    return sorted(arrays)
 
 
 def _jsonable(o):
@@ -367,6 +392,10 @@ def _run_ours(a, real_stdout):
     barrier()
     launches = int(L.wsp_launch_count() - launches0)
     clocks = sampler.stop()
+    if a.dump_outputs:
+        # read before the instrumented decoder pass below overwrites the logits
+        names = dump_outputs(a.dump_outputs, {"tokens": toks_r, "logits": ctx.logits(B)}, "" if world == 1 else "rank%d_" % rank)
+        print("[bench] wrote %s to %s" % (", ".join(n + ".npy" for n in names), a.dump_outputs), flush=True)
     val_ms = max_over_ranks(val_ms_dev)
     match_fixture = None
     if fixture_tokens is not None:

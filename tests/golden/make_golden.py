@@ -8,6 +8,7 @@ Inputs are fully determined by whisper_b200/synth.py (model seed 1234, PCM chunk
 tensors are stored as deterministic sub-samples to keep the fixtures small.
 
     python tests/golden/make_golden.py            # rewrites tests/golden/*.npz
+    python tests/golden/make_golden.py --sampler  # tests/golden/sampler.npz: needs a B200 besides oracle/_ref
 """
 import ctypes as C
 import os
@@ -276,6 +277,39 @@ def make_real_shapes(models=None):
     return out
 
 
+# A model shape and clip no other fixture covers (tests/test_gpu_parity.py::test_live_reference_when_prebuilt): log-mel, cross-attention
+# keys and the greedy tokens of the bench loop at the reference's default 4 threads.
+LIVE_MODEL, LIVE_CHUNK, LIVE_STEPS = "tiny.en-sc", 5, 20
+
+
+def make_live():
+    o = RefOracle(synth.model_path(LIVE_MODEL), threads=4)
+    pcm = synth.synth_pcm(LIVE_CHUNK)
+    mel = o.pcm_to_mel(pcm)
+    o.encode(0)
+    ck, _ = o.cross_kv()
+    prompt = prompt_of(o)
+    _, toks, _ = o.bench_chunk(pcm, prompt, LIVE_STEPS)
+    return {"mel_shape": np.array(mel.shape, np.int32), "mel": mel[:, ::MEL_STEP].astype(np.float32),
+            "cross_k": ck[:, ::ROW_STEP].astype(np.float16), "prompt": np.array(prompt, np.int32), "tokens": np.asarray(toks, np.int32)}
+
+
+def make_sampler():
+    """The reference's whisper_sample_best / whisper_sample_timestamp (ora_sample_from_probs) on the probability rows the GPU sampler's
+    softmax makes of tests/test_gpu_sampler.make_rows(), in row order.  Needs a B200 and oracle/_ref on the same machine."""
+    from tests.test_gpu_sampler import MODEL, SPECIAL4, make_rows
+    from whisper_b200 import capi
+    o = RefOracle(synth.model_path(MODEL), threads=1)
+    res = {k: [] for k in ("id", "tid", "p", "pt", "ptsum")}
+    for lg, force_ts, initial, _label in make_rows():
+        probs, _ = capi.test_sample(lg, SPECIAL4, force_ts, initial)
+        for row in probs:
+            s = o.sample_from_probs(row, force_ts, initial)
+            for k in res:
+                res[k].append(s[k])
+    return {k: np.array(v, np.int32 if k in ("id", "tid") else np.float32) for k, v in res.items()}
+
+
 TOKENIZER_TEXTS = [b" hello hellox 12345!", b" hello world's , worlds 345 12", b" t12 t345", b""]
 
 
@@ -310,11 +344,18 @@ if __name__ == "__main__":
     if "--lang" in sys.argv:
         save("lang_detect", make_lang())
         sys.exit(0)
+    if "--live" in sys.argv:
+        save("tiny_en_live", make_live())
+        sys.exit(0)
+    if "--sampler" in sys.argv:
+        save("sampler", make_sampler())
+        sys.exit(0)
     if "--cases" in sys.argv:
         for name in [a for a in sys.argv[1:] if not a.startswith("--")] or list(CASES):
             save(name, make(*CASES[name]))
         sys.exit(0)
     save("full_runs", make_full())
     save("lang_detect", make_lang())
+    save("tiny_en_live", make_live())
     for name, (model, chunk, n, off) in CASES.items():
         save(name, make(model, chunk, n, off))

@@ -14,6 +14,8 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 N_SIGNALS = 16
+# a second, disjoint set of signals, recorded the same way (tests/test_vad.py::test_detector_matches_live_reference)
+HELD_OUT_SEEDS = range(100, 130)
 
 
 def vad_signal(seed: int, secs: int = 12) -> np.ndarray:
@@ -68,7 +70,7 @@ def drive(lib, prefix: str, seed: int):
 if __name__ == "__main__":
     ref = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "liboracle_vad.so"))
     data = {}
-    for seed in range(N_SIGNALS):
+    for seed in list(range(N_SIGNALS)) + list(HELD_OUT_SEEDS):
         res = drive(ref, "ora_vad", seed)
         data["s%d" % seed] = np.asarray(res, np.int64)
         print(seed, "calls", len(res), "distinct results", len(set(res)), "last", res[-1])

@@ -1,7 +1,6 @@
 """Parity of the CUDA hot path with the reference, on a B200, through the C ABI.
 
-Oracle: the committed fixtures tests/golden/*.npz (outputs of oracle/_ref = the reference's unmodified CPU code), plus oracle/_ref
-itself when the prebuilt library travelled to this box.  Nothing here reads /root/reference.
+Oracle: the committed fixtures tests/golden/*.npz (outputs of oracle/_ref = the reference's unmodified CPU code).
 
 Tolerances (floating point, activations O(1), logits rms ~3):
   mel 5e-4 · encoder tensors 8e-3 · f16 KV memories 4e-3 · logits 3e-2 (measured: 1e-4, 3e-3, 2e-3, 1e-2).
@@ -225,26 +224,24 @@ def test_step_kernels_agree_for_every_thread_count(threads):
 
 
 def test_live_reference_when_prebuilt():
-    """If oracle/_ref travelled to this box, compare against the reference live on a case that has no committed fixture."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not present")
-    m, e, c = open_model("tiny.en-sc")
-    o = ref.RefOracle(synth.model_path("tiny.en-sc"), threads=4)
-    pcm = synth.synth_pcm(5)
-    mel_ref = o.pcm_to_mel(pcm)
+    """A model shape and clip that the parity cases above do not cover (tiny.en-sc, chunk 5): log-mel, cross-attention keys and 20 greedy
+    tokens against the reference's (tests/golden/tiny_en_live.npz, make_golden.py --live)."""
+    from tests.golden.make_golden import LIVE_CHUNK, LIVE_MODEL, LIVE_STEPS
+    g = golden("tiny_en_live")
+    m, e, c = open_model(LIVE_MODEL)
+    pcm = synth.synth_pcm(LIVE_CHUNK)
     c.pcm_to_mel(0, pcm)
-    assert np.abs(c.get_mel(0) - mel_ref).max() < TOL_MEL
-    o.encode(0)
+    mel = c.get_mel(0)
+    assert mel.shape == tuple(g["mel_shape"])
+    assert np.abs(mel[:, ::MEL_STEP] - g["mel"]).max() < TOL_MEL
     c.encode(1)
-    ck, cv = o.cross_kv()
     d, T, H, L = m.n_audio_state, m.n_audio_ctx, m.n_audio_head, m.n_text_layer
     got = c.get_tensor("cross_k").reshape(L, H, T, 64).transpose(0, 2, 1, 3).reshape(L, T, d)
-    assert np.abs(got - ck).max() < TOL_KV * synth.SC_ENC_GAIN_CALIBRATED
+    assert np.abs(got[:, ::ROW_STEP] - g["cross_k"].astype(np.float32)).max() < TOL_KV * synth.SC_ENC_GAIN_CALIBRATED
     prompt = m.prompt_init()
-    ref_s, ref_toks, _ = o.bench_chunk(pcm, prompt, 20)
-    toks, _ = c.run_chunks([pcm], prompt, 20)
-    assert toks[0].tolist() == ref_toks.tolist()
+    assert prompt == g["prompt"].tolist()
+    toks, _ = c.run_chunks([pcm], prompt, LIVE_STEPS)
+    assert toks[0].tolist() == g["tokens"].tolist()
 
 
 @pytest.mark.parametrize("model", ["tiny.en-sc", "base.en-sc", "medium-sc", "large-sc"])

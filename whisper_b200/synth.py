@@ -11,6 +11,7 @@ from __future__ import annotations
 
 import os
 import struct
+import tempfile
 from dataclasses import dataclass
 
 import numpy as np
@@ -410,8 +411,9 @@ def write_script_model(path: str, base: str, seed: int = 1234, stage: int = 2, c
 
 
 def model_path(name: str, seed: int = 1234, cache_dir: str | None = None) -> str:
-    """Return (creating on first use) the cached synthetic model file for `name`."""
-    cache_dir = cache_dir or os.environ.get("WSP_MODEL_CACHE", "/tmp/wsp_models")
+    """Return (creating on first use) the cached synthetic model file for `name`.  The default cache is per user under the system's
+    temporary directory: on a shared host another user's cache would be unwritable, and its files not ours to trust."""
+    cache_dir = cache_dir or os.environ.get("WSP_MODEL_CACHE") or os.path.join(tempfile.gettempdir(), "wsp_models-%d" % os.getuid())
     os.makedirs(cache_dir, exist_ok=True)
     p = os.path.join(cache_dir, "ggml-%s-synth%d%s.bin" % (name, seed, "-r2" if name.endswith(("-sc", "-sc1")) else ""))
     if not os.path.exists(p):
