@@ -175,8 +175,14 @@ wsp_status wsp_timer_stop( wsp_context* c, float* ms );
  * around every launch.  kinds: 0 skinny GEMM, 1 cross-attention, 2 self-attention, 3 other (embedding, sampler) */
 wsp_status wsp_profile_decode( wsp_context* c, int32_t batch, int32_t n_steps, float ms_by_kind[ 4 ], int32_t launches_by_kind[ 4 ] );
 
-/* test hook: named intermediates as f32.  Names: "mel", "enc.conv1" ([3000][d] after GELU), "enc.x0" ([1500][d] input of layer 0),
- * "enc.layers" (residual stream after the last layer), "encode-out" (ln_post, f16-rounded), "cross_k", "cross_v" ([L][T][d] of slot 0). */
+/* test hook: named intermediates of chunk `slot` as f32.  Names:
+ *   "mel" ([80][n_len]), "enc.input" ([3000][80] f16 encoder input), "enc.conv1" ([3000][d] after GELU),
+ *   "enc.x" ([T][d] residual stream: input of layer 0, or the output of the last layer run, see wsp_debug_set_encoder_layers),
+ *   "encode-out" / "enc.xn" ([T][d] ln_post, f16-rounded), "enc.q", "enc.k" ([H][T][64] of the last layer run), "enc.vt" ([H][64][T
+ *   padded]), "enc.attn" ([T][d] attention output of the last layer run),
+ *   "cross_k", "cross_v" ([L][H][T][64] cross-attention memories), "self_k", "self_v" ([L][H][n_text_ctx][64] self-KV cache; rows
+ *   at and past the decoder's n_past hold whatever earlier calls wrote there),
+ *   "dec.x" ([8][d] first rows of the decoder's residual stream, for any slot; step mode 2 does not write it). */
 wsp_status wsp_get_tensor( wsp_context* c, const char* name, int32_t slot, float* dst, size_t cap_floats, size_t* n_floats );
 /* debug: run only the first n encoder layers (negative = all) */
 wsp_status wsp_debug_set_encoder_layers( wsp_context* c, int32_t n );

@@ -300,21 +300,24 @@ wsp_status wsp_get_tensor( wsp_context* cc, const char* name, int32_t slot, floa
 	else if( nm == "enc.q" ) { f16 = c.q + (size_t)slot * T * d; n = (size_t)T * d; }                                             // [H][T][64]
 	else if( nm == "enc.k" ) { f16 = c.k + (size_t)slot * T * d; n = (size_t)T * d; }
 	else if( nm == "enc.vt" ) { f16 = c.vt + (size_t)slot * H * 64 * c.Tp; n = (size_t)H * 64 * c.Tp; }                            // [H][64][Tp]
-	else if( nm == "cross_k" || nm == "cross_v" )
+	else if( nm == "cross_k" || nm == "cross_v" || nm == "self_k" || nm == "self_v" )
 	{
-		// gathered per layer below: [L][H][T][64] of this slot
-		n = (size_t)L * T * d;
+		// gathered per layer below: [L][H][rows][64] of this slot, rows = T (cross-attention memories) or n_text_ctx (self-KV cache)
+		const bool self = nm[ 0 ] == 's';
+		const size_t per = (size_t)( self ? hp.n_text_ctx : T ) * hp.n_text_state;
+		n = (size_t)L * per;
 		if( n_floats ) *n_floats = n;
 		if( !dst ) return WSP_OK;
 		if( cap < n ) return fail( WSP_E_BOUNDS, "dst too small" );
 		DevTmp<float> tmp;
-		WSP_CUDA( tmp.alloc( (size_t)T * d ) );
-		const __half* base = nm == "cross_k" ? c.crossK : c.crossV;
+		WSP_CUDA( tmp.alloc( per ) );
+		const __half* base = nm == "cross_k" ? c.crossK : nm == "cross_v" ? c.crossV : nm == "self_k" ? c.selfK : c.selfV;
 		for( int l = 0; l < L; l++ )
 		{
-			const __half* src = base + ( (size_t)l * c.maxB + slot ) * T * d;
-			half_to_float_kernel<<<(unsigned)( ( (size_t)T * d + 255 ) / 256 ), 256>>>( src, tmp.p, (size_t)T * d );
-			WSP_CUDA( cudaMemcpy( dst + (size_t)l * T * d, tmp.p, (size_t)T * d * 4, cudaMemcpyDeviceToHost ) );
+			const __half* src = base + ( (size_t)l * c.maxB + slot ) * per;
+			half_to_float_kernel<<<(unsigned)( ( per + 255 ) / 256 ), 256, 0, c.stream>>>( src, tmp.p, per );
+			WSP_CUDA( cudaMemcpyAsync( dst + (size_t)l * per, tmp.p, per * 4, cudaMemcpyDeviceToHost, c.stream ) );
+			WSP_CUDA( cudaStreamSynchronize( c.stream ) );
 		}
 		return WSP_OK;
 	}
